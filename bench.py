@@ -63,6 +63,8 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="headline step only (no downsample / merge / tiles / fixtures / all-gather side measurements)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0) to DIR/<name>.npy; see dump_outputs()")
     return ap.parse_args()
 
 
@@ -574,6 +576,53 @@ def run_fetch_e2e(args, codec, ts, vals, start, P, rank, world, dev, barrier, di
             "api": "m3tsz_fetch_batch_host (H2D compressed replicas -> decode -> series merge -> D2H merged)"}
 
 
+DUMP_SEED = 20240601
+DUMP_MAX_SCALAR_SERIES = 1 << 20
+DUMP_MAX_ROW_SERIES = 256
+
+
+def dump_outputs(out_dir, enc, dec_pm, start):
+    """Writes the results of the timed step (encode into per-series segments, then point-major
+    decode of them) as float32 / float64 .npy files under out_dir, so that two builds can be
+    compared output for output on the same seeded batch.  Under 64 MB in all:
+
+      series_index         [K]     the series whose full rows are written: a fixed seeded sample
+      encode_segments      [K, B]  their compressed segments, one byte per element, zero past out_len
+      decode_ts_offset_ns  [P, K]  their decoded timestamps minus the series start (exact in float64)
+      decode_values        [P, K]  their decoded values
+      encode_out_len, encode_status, decode_n_points, decode_status, decode_unit
+                           [M]     per series, for the first M = min(S, 2^20) series
+    """
+    import numpy as np
+    import torch
+    P, S = dec_pm.values.shape
+    B = enc.out.shape[1]
+    K = min(S, DUMP_MAX_ROW_SERIES, max(1, (32 << 20) // (P * 16 + B * 4)))
+    M = min(S, DUMP_MAX_SCALAR_SERIES)
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(S, size=K, replace=False))
+    idx = torch.from_numpy(rows).to(enc.out.device)
+    seg = enc.out[idx]
+    seg = seg * (torch.arange(B, device=seg.device)[None, :] < enc.out_len[idx][:, None])
+    arrays = {
+        "series_index": rows.astype(np.float64),
+        "encode_segments": seg.to(torch.float32),
+        "decode_ts_offset_ns": (dec_pm.ts[:, idx] - start[idx][None, :]).to(torch.float64),
+        "decode_values": dec_pm.values[:, idx],
+        "encode_out_len": enc.out_len[:M].to(torch.float64),
+        "encode_status": enc.status[:M].to(torch.float32),
+        "decode_n_points": dec_pm.n_points[:M].to(torch.float64),
+        "decode_status": dec_pm.status[:M].to(torch.float32),
+        "decode_unit": dec_pm.unit[:M].to(torch.float32),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else a
+        total += a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+    assert total <= 64 << 20, total
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -676,6 +725,8 @@ def run_ours(args):
     ms_total, dec_ms_max = float(t[0]), float(t[1])
     ms_per_step = ms_total / args.steps
     value = S * P * world / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:  # before the timings below reuse enc and dec_pm
+        dump_outputs(args.dump_outputs, enc, dec_pm, start)
 
     # separate per-kernel timings (same buffers, outside the headline region)
     def time_fn(fn, n=5):

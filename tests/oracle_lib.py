@@ -21,7 +21,8 @@ ERR_DOD_OVERFLOW = 4
 
 def build_oracle(force=False):
     srcs = [os.path.join(ORACLE_DIR, f) for f in ("m3tsz_oracle.c", "m3tsz_merge_oracle.c",
-                                                  "m3tsz_segment_oracle.c", "m3tsz_oracle.h")]
+                                                  "m3tsz_segment_oracle.c", "m3tsz_query_oracle.c",
+                                                  "m3tsz_oracle.h")]
     if (not force and os.path.exists(_LIB_PATH)
             and os.path.getmtime(_LIB_PATH) >= max(os.path.getmtime(f) for f in srcs)):
         return _LIB_PATH
